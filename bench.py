@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo (libzkb200.so, sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm on the host cores, SAME circuit
     python bench.py --curve bls12_381 --log-n 22 --gpus 8    # BASELINE.json config 4
+    python bench.py --steps K --dump-outputs DIR             # also write the proof of the last timed step under DIR
 
 Workload (default = BASELINE.json config 3): synthetic R1CS with 2^20 - 2 constraints, one public input, so the
 evaluation domain is exactly 2^20; uniform 252-bit witness (MSM worst case), BN254.  A "step" is one proof:
@@ -126,6 +127,15 @@ class CpuFieldOps:
         return self.oc.field_op(self.cid, field, op, a, b)
 
 
+def dump_outputs(out_dir, proof, fq_bytes):
+    """The proof a caller receives (A in G1, B in G2, C in G1) as DIR/proof_{a,b,c}.npy.  A coordinate is a 256- or
+    384-bit field element, so it is stored as 16-bit little-endian limbs in float64, which hold it exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    limbs = np.frombuffer(proof, dtype="<u2").astype(np.float64).reshape(8, fq_bytes // 2)
+    for name, arr in (("proof_a", limbs[0:2]), ("proof_b", limbs[2:6].reshape(2, 2, -1)), ("proof_c", limbs[6:8])):
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def workload_name(args):
     return f"synthetic-r1cs-2^{args.log_n}-{args.curve}-groth16"
 
@@ -167,6 +177,8 @@ def run_reference(args):
         dt = time.perf_counter() - t
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof, fq_bytes)
     total = sum(times)
     value = n_cons * len(times) / total
     line = {
@@ -200,7 +212,10 @@ def main():
     ap.add_argument("--table-c", type=int, default=0, help="force the window width of the HBM window tables (0: cost model)")
     ap.add_argument("--opt", action="append", default=[], metavar="ID=VALUE", help="zkb_ctx_set_option(ID, VALUE) before the key is loaded (tuning runs)")
     ap.add_argument("--pipeline", type=int, default=2, choices=[1, 2], help="proofs in flight per GPU (2: submit i+1 before collecting i)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step as DIR/proof_{a,b,c}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)          # timing rule: at least three warm-up steps, in both arms
     if args.impl == "reference":
         return run_reference(args)
@@ -355,6 +370,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0 and proof != proof2:
         raise SystemExit("resident and e2e proofs differ")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof, ctx.fq_bytes)
     # latency of ONE proof with nothing else in flight (what --pipeline 1 would time), after the throughput runs
     lat = []
     saved_depth = args.pipeline
