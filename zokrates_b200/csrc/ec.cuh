@@ -6,6 +6,10 @@
 // mixed addition 8M + 2S (= 10 field multiplications, the SURVEY.md §8d accounting unit), full
 // addition 12M + 2S, doubling 6M + 3S.  Results are representation independent: the affine point
 // is canonical, so outputs are bit-identical to any other correct implementation.
+//
+// Y3 = R (Q - X3) - Y PPP is one F::mul_sub: both products unreduced, one Montgomery reduction.  The
+// Pd / Rd zero tests below are exact only because every field operation returns the canonical
+// residue (< p), never a merely congruent value.
 #pragma once
 #include "fp2.cuh"
 
@@ -40,7 +44,7 @@ struct XYZZ {
     F X2 = F::sqr(p.x);
     F M = F::add(F::dbl(X2), X2);
     F X3 = F::sub(F::sqr(M), F::dbl(S));
-    F Y3 = F::sub(F::mul(M, F::sub(S, X3)), F::mul(W, p.y));
+    F Y3 = F::mul_sub(M, F::sub(S, X3), W, p.y);
     return XYZZ{X3, Y3, V, W};
   }
 
@@ -52,7 +56,7 @@ struct XYZZ {
     F X2 = F::sqr(p.x);
     F M = F::add(F::dbl(X2), X2);
     F X3 = F::sub(F::sqr(M), F::dbl(S));
-    F Y3 = F::sub(F::mul(M, F::sub(S, X3)), F::mul(W, p.y));
+    F Y3 = F::mul_sub(M, F::sub(S, X3), W, p.y);
     return XYZZ{X3, Y3, F::mul(V, p.zz), F::mul(W, p.zzz)};  // identity stays identity (ZZ = 0)
   }
 
@@ -72,7 +76,7 @@ struct XYZZ {
     F PPP = F::mul(Pd, PP);
     F Q = F::mul(a.x, PP);
     F X3 = F::sub(F::sub(F::sqr(Rd), PPP), F::dbl(Q));
-    F Y3 = F::sub(F::mul(Rd, F::sub(Q, X3)), F::mul(a.y, PPP));
+    F Y3 = F::mul_sub(Rd, F::sub(Q, X3), a.y, PPP);
     return XYZZ{X3, Y3, F::mul(a.zz, PP), F::mul(a.zzz, PPP)};
   }
 
@@ -94,7 +98,7 @@ struct XYZZ {
     F PPP = F::mul(Pd, PP);
     F Q = F::mul(U1, PP);
     F X3 = F::sub(F::sub(F::sqr(Rd), PPP), F::dbl(Q));
-    F Y3 = F::sub(F::mul(Rd, F::sub(Q, X3)), F::mul(S1, PPP));
+    F Y3 = F::mul_sub(Rd, F::sub(Q, X3), S1, PPP);
     return XYZZ{X3, Y3, F::mul(F::mul(a.zz, b.zz), PP), F::mul(F::mul(a.zzz, b.zzz), PPP)};
   }
 

@@ -72,6 +72,54 @@ struct alignas(16) Fp64 {
     return (t[N] || geq_p(o)) ? sub_p(o) : o;
   }
   ZKB_HD static Fp64 sqr(const Fp64& a) { return mul(a, a); }
+  ZKB_HD static Fp64 mul_sub(const Fp64& a, const Fp64& b, const Fp64& c, const Fp64& d) { return sub(mul(a, b), mul(c, d)); }
+
+  // the lazy-reduction interface of Fp<P> (used by Fp2T): unreduced 2N-limb products and one reduction per sum
+  struct Wide {
+    uint64_t v[2 * N];
+  };
+  ZKB_HD static Fp64 add_raw(const Fp64& a, const Fp64& b) {
+    Fp64 t; uint64_t c = 0;
+    for (int i = 0; i < N; i++) { u128 s = (u128)a.v[i] + b.v[i] + c; t.v[i] = (uint64_t)s; c = (uint64_t)(s >> 64); }
+    return t;
+  }
+  ZKB_HD static Wide mul_wide(const Fp64& a, const Fp64& b) {
+    Wide t;
+    for (int i = 0; i < 2 * N; i++) t.v[i] = 0;
+    for (int i = 0; i < N; i++) {
+      uint64_t c = 0;
+      for (int j = 0; j < N; j++) { u128 s = (u128)a.v[j] * b.v[i] + t.v[i + j] + c; t.v[i + j] = (uint64_t)s; c = (uint64_t)(s >> 64); }
+      t.v[i + N] = c;
+    }
+    return t;
+  }
+  ZKB_HD static Wide sqr_wide(const Fp64& a) { return mul_wide(a, a); }
+  ZKB_HD static Fp64 redc(const Wide& T) {  // T < p R
+    uint64_t t[2 * N + 1];
+    for (int i = 0; i < 2 * N; i++) t[i] = T.v[i];
+    t[2 * N] = 0;
+    const uint64_t inv = inv64();
+    for (int i = 0; i < N; i++) {
+      const uint64_t m = t[i] * inv;
+      uint64_t c = 0;
+      for (int j = 0; j < N; j++) { u128 s = (u128)m * modl(j) + t[i + j] + c; t[i + j] = (uint64_t)s; c = (uint64_t)(s >> 64); }
+      for (int k = i + N; c && k <= 2 * N; k++) { u128 s = (u128)t[k] + c; t[k] = (uint64_t)s; c = (uint64_t)(s >> 64); }
+    }
+    Fp64 o; for (int i = 0; i < N; i++) o.v[i] = t[N + i];
+    return (t[2 * N] || geq_p(o)) ? sub_p(o) : o;
+  }
+  ZKB_HD static Wide add_wide(const Wide& a, const Wide& b) {
+    Wide t; uint64_t c = 0;
+    for (int i = 0; i < 2 * N; i++) { u128 s = (u128)a.v[i] + b.v[i] + c; t.v[i] = (uint64_t)s; c = (uint64_t)(s >> 64); }
+    return t;
+  }
+  ZKB_HD static Wide sub_wide(const Wide& a, const Wide& b) {
+    Wide t; uint64_t borrow = 0;
+    for (int i = 0; i < 2 * N; i++) { u128 d = (u128)a.v[i] - b.v[i] - borrow; t.v[i] = (uint64_t)d; borrow = (uint64_t)(d >> 64) & 1; }
+    return t;
+  }
+  ZKB_HD static Wide p2() { Wide t; for (int i = 0; i < 2 * N; i++) t.v[i] = ((uint64_t)P::p2(2 * i + 1) << 32) | P::p2(2 * i); return t; }
+  ZKB_HD static Wide p2x2() { Wide t; for (int i = 0; i < 2 * N; i++) t.v[i] = ((uint64_t)P::p2x2(2 * i + 1) << 32) | P::p2x2(2 * i); return t; }
   ZKB_HD static Fp64 mul_ni(const Fp64& a, const Fp64& b) { return mul(a, b); }
   ZKB_HD static Fp64 to_mont(const Fp64& a) { return mul(a, r2()); }
   ZKB_HD static Fp64 from_mont(const Fp64& a) { Fp64 o = zero(); o.v[0] = 1; return mul(a, o); }
